@@ -4,6 +4,7 @@ denoised tokens/sec (text+image) per 512x512 @ 64-step sample, variant A 8B, cfg
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path
     python bench.py --impl reference ...                            # the reference algorithm on the host CPU (oracle port)
+    python bench.py --dump-outputs DIR ...                          # also writes what the last timed sample computed (.npy)
 
 One "step" = one full sample = one generate_ti2ti call: 128 denoising iterations, 192 transformer forwards
 (128 conditional + 64 unconditional-image), 128 text steps, 64 image steps -> 1280 denoised tokens.
@@ -21,6 +22,7 @@ import os
 import statistics
 import subprocess
 import sys
+import tempfile
 import time
 
 import torch
@@ -74,11 +76,11 @@ class ClockSampler:
          "clocks_event_reasons.sw_thermal_slowdown,clocks_event_reasons.sw_power_cap")
 
     def __init__(self, gpu_index: int):
-        self.idx, self.p, self.path = gpu_index, None, f"/tmp/mmdp_clocks_{os.getpid()}.csv"
+        self.idx, self.p = gpu_index, None
 
     def start(self):
         try:
-            self.f = open(self.path, "w")
+            self.f = tempfile.NamedTemporaryFile("w+", prefix="mmdp_clocks_", suffix=".csv")
             self.p = subprocess.Popen(["nvidia-smi", f"--query-gpu={self.Q}", "--format=csv,noheader,nounits", "-lms", "200",
                                        "-i", str(self.idx)], stdout=self.f, stderr=subprocess.DEVNULL)
         except Exception:
@@ -92,9 +94,11 @@ class ClockSampler:
             self.p.wait(timeout=5)
         except Exception:
             self.p.kill()
-        self.f.close()
+        self.f.seek(0)
+        lines = self.f.readlines()
+        self.f.close()  # removes the file
         sm, mx, reasons, power = [], [], set(), []
-        for line in open(self.path):
+        for line in lines:
             c = [x.strip() for x in line.split(",")]
             if len(c) < 8:
                 continue
@@ -639,11 +643,32 @@ def measure_tensor_parallel(args, model_cfg, device, rank, world, replica_model,
                                      "single-GPU forward with the 1-CTA GEMM kernel instead of the CTA-pair kernel"}}
 
 
+DUMP_MAX_ELEMENTS = 1 << 22  # per array: 16 MB of float32
+
+
+def dump_outputs(out_dir: str, st) -> None:
+    """Writes what the last timed sample computed as `out_dir/<name>.npy`, for comparing two builds output for output:
+    `ids` is the final id buffer denoise_loop returns (float64, exact for token ids); `text_logits` and `image_logits` are the
+    buffers of the sample's last conditional forward (text rows x vocabulary, VQ rows x codebook), as float32. An array with
+    more than DUMP_MAX_ELEMENTS elements is written as a fixed, seeded sample of its flattened elements (the same positions
+    in every run)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in (("ids", st.ids.double()), ("text_logits", st.text_logits.float()), ("image_logits", st.cond_vq.float())):
+        flat = t.reshape(-1)
+        if flat.numel() > DUMP_MAX_ELEMENTS:
+            keep = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_MAX_ELEMENTS].sort().values
+            t = flat[keep.to(flat.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=2)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=2, help="timed samples")
+    ap.add_argument("--warmup", type=int, default=3, help="untimed samples before them")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed samples, write what the last one computed as DIR/<name>.npy "
+                    "(rank 0)")
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--tiny", action="store_true", help="2-layer d=256 model: plumbing check only (INVALID as a benchmark number)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
@@ -658,6 +683,10 @@ def main():
     ap.add_argument("--tp", action="store_true", help="N > 1: ONE sample tensor-parallel over the N GPUs (strong scaling, NCCL "
                     "all-reduce) instead of N independent replicas")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and (args.impl != "b200" or args.variant != "a"):
+        ap.error("--dump-outputs writes the outputs of the variant A path of --impl b200")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -747,6 +776,8 @@ def main():
             prof = _lib.prof_summary()
             _lib.lib.mmdp_prof_enable(0)
         barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, states[-1])
 
     # ---- sub-records on the other BASELINE configs (every rank takes part where a collective or a barrier is involved)
     extras = {}
